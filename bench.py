@@ -13,6 +13,7 @@ Workloads (BASELINE.json configs):
   --config c3       emit the configs[2] line as the main line on one GPU
 
   python bench.py [--gpus N] [--steps K] [--warmup W]            our CUDA path
+  python bench.py ... --dump-outputs DIR                          also write the last timed step's outputs as DIR/*.npy
   python bench.py --impl reference ...                            the CPU path: cv2 (OpenCV) tracker twin + oracle estimator
 Under torchrun (N > 1) rank 0 prints ONE JSON line.
 """
@@ -131,6 +132,26 @@ class ClockSampler:
         reasons = sorted({name for r in rows for bit, name in self.REASONS.items() if r[2] & bit})
         return {"sm_mhz": float(np.median(sm)) if sm else None, "sm_max_mhz": self.max_mhz, "reasons": reasons,
                 "samples": len(sm), "source": "NVML, polled every 2 ms inside the timed region"}
+
+
+def step_outputs(ids, obs, est):
+    """What a caller of the single-sequence path holds after a step: the feature message the tracker published (ids; x, y,
+    z, u, v, vx, vy per feature) and the estimator's window after processImage (p, q wxyz, v, ba, bg per frame; td)."""
+    states, td = est.states()
+    return {"feature_ids": np.asarray(ids, np.float64), "feature_obs": np.asarray(obs, np.float64),
+            "window_states": np.asarray(states, np.float64), "window_td": np.array([td], np.float64)}
+
+
+def dump_outputs(directory, arrays):
+    """--dump-outputs: one float64 .npy file per array, for output-by-output comparison of two builds."""
+    os.makedirs(directory, exist_ok=True)
+    for name, arr in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), np.asarray(arr, np.float64))
+
+
+def check_steps(done, wanted, what):
+    if done != wanted:
+        raise RuntimeError(f"{what}: {done} timed steps instead of the {wanted} asked for (the rendered sequence ran out)")
 
 
 def make_gpu_pair(device):
@@ -258,7 +279,7 @@ def run_ours_pass(seq, ts, imgs, imu, n_init, warmup, steps, device, host_images
             return produce()
 
     stage = Serial() if profile else TwoStage(produce, n_init + warmup, n_pub)
-    pubs, first_msg, n_timed, started = 0, True, 0, False
+    pubs, first_msg, n_timed, started, last_msg = 0, True, 0, False, None
     while pubs < n_pub:
         timed = pubs >= n_init + warmup
         if timed and not started:
@@ -286,6 +307,7 @@ def run_ours_pass(seq, ts, imgs, imu, n_init, warmup, steps, device, host_images
             launches += step_launch
             h2d += step_h2d
             d2h += step_d2h
+            last_msg = (ids, d)
         if est.info()["solver_flag"] == 1:
             st, _ = est.states()
             traj_t.append(stamp)
@@ -293,8 +315,10 @@ def run_ours_pass(seq, ts, imgs, imu, n_init, warmup, steps, device, host_images
         pubs += 1
     region_ms = gate.end() if started else 0.0
     stage.go()
+    check_steps(n_timed, steps, "single-sequence pass")
     times = [region_ms / max(n_timed, 1)] * n_timed if started else []
-    out = dict(times=times, launches=launches, h2d=h2d, d2h=d2h, traj_t=traj_t, traj_p=traj_p, info=est.info())
+    out = dict(times=times, launches=launches, h2d=h2d, d2h=d2h, traj_t=traj_t, traj_p=traj_p, info=est.info(),
+               outputs=step_outputs(*last_msg, est) if last_msg else {})
     if profile:
         out["trk_k"], out["est_k"] = trk.kernel_times(), est.kernel_times()
     trk.close()
@@ -372,13 +396,16 @@ def run_batch_pass(inputs, n_seq, n_init, warmup, steps, device, host_images=Fal
     gate.begin()
     frames = ses.advance(steps)
     region_ms = gate.end()
+    check_steps(frames, steps * n_seq, f"batched pass ({n_seq} sequences x {steps} steps)")
     after = [ses.stats(k) for k in range(n_seq)]
     trajs = [ses.trajectory(k) for k in range(n_seq)]
     infos = [m.info() for m in eb.members]
+    windows = [m.states() for m in eb.members]
+    outputs = {"window_states": np.stack([w[0] for w in windows]), "window_td": np.array([w[1] for w in windows], np.float64)}
     out = dict(frames=frames, region_ms=region_ms, fps=frames / (region_ms / 1e3) if region_ms else 0.0,
                launches=sum(a_["launches"] - b_["launches"] for a_, b_ in zip(after, before)),
                h2d=sum(a_["h2d"] - b_["h2d"] for a_, b_ in zip(after, before)),
-               d2h=sum(a_["d2h"] - b_["d2h"] for a_, b_ in zip(after, before)), trajs=trajs, infos=infos)
+               d2h=sum(a_["d2h"] - b_["d2h"] for a_, b_ in zip(after, before)), trajs=trajs, infos=infos, outputs=outputs)
     out["est_groups"] = eb.groups()
     if profile:
         out["trk_k"], out["est_k"] = tb.kernel_times(), eb.kernel_times()
@@ -441,7 +468,7 @@ def run_reference_pass(seq, ts, imgs, imu, n_init, warmup, steps, front="cv2"):
         return float(ts[cursor[0] - 1]), ids, d
 
     stage = TwoStage(produce, n_init + warmup, n_pub)
-    pubs, first_msg, n_timed, t0 = 0, True, 0, None
+    pubs, first_msg, n_timed, t0, last_msg = 0, True, 0, None, None
     t_back = 0.0
     while pubs < n_pub:
         if pubs == n_init + warmup:
@@ -461,6 +488,7 @@ def run_reference_pass(seq, ts, imgs, imu, n_init, warmup, steps, front="cv2"):
         if t0 is not None:
             n_timed += 1
             t_back += time.perf_counter() - tb0
+            last_msg = (ids, d)
         if est.info()["solver_flag"] == 1:
             st, _ = est.states()
             traj_t.append(stamp)
@@ -468,8 +496,10 @@ def run_reference_pass(seq, ts, imgs, imu, n_init, warmup, steps, front="cv2"):
         pubs += 1
     total_ms = (time.perf_counter() - t0) * 1e3 if t0 is not None else 0.0
     stage.go()
+    check_steps(n_timed, steps, "reference pass")
     return dict(times=[total_ms / max(n_timed, 1)] * n_timed, traj_t=traj_t, traj_p=traj_p, front=used,
-                front_ms_per_frame=1e3 * t_front[0] / max(n_timed, 1), back_ms_per_frame=1e3 * t_back / max(n_timed, 1))
+                front_ms_per_frame=1e3 * t_front[0] / max(n_timed, 1), back_ms_per_frame=1e3 * t_back / max(n_timed, 1),
+                outputs=step_outputs(*last_msg, est) if last_msg else {})
 
 
 def _reference_worker(args):
@@ -564,6 +594,9 @@ def main():
     ap.add_argument("--seqs-per-gpu", type=int, default=SEQS_PER_GPU, help="members of the batched workload (configs[2]/[4])")
     ap.add_argument("--distinct", type=int, default=16, help="distinct rendered sequences behind the batch members")
     ap.add_argument("--no-c3", action="store_true", help="skip the configs[2] object of the single-GPU line")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the timed path returned in its last step as DIR/<name>.npy (float64): for one sequence the "
+                         "feature message and the estimator window, for a batch every member's window (rank 0's members)")
     a = ap.parse_args()
     rank, world, local = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1)), int(os.environ.get("LOCAL_RANK", 0))
     warmup = max(a.warmup, 3) if a.impl == "b200" else a.warmup
@@ -575,6 +608,8 @@ def main():
         INIT_PUBS, WORKLOAD = 22, WORKLOAD_C4
         a.no_c3 = True
     batched = a.config == "c3" or (a.config == "auto" and world > 1)
+    if a.dump_outputs and a.impl == "reference" and batched:
+        ap.error("--dump-outputs: the reference arm writes outputs of the single-sequence workload only")
     S = a.seqs_per_gpu
     n_distinct = max(1, min(a.distinct, S))
 
@@ -585,6 +620,8 @@ def main():
         if not batched:
             seq, ts, imgs, imu = sequence_inputs(0, INIT_PUBS + warmup + a.steps)
             r = run_reference_pass(seq, ts, imgs, imu, INIT_PUBS, warmup, a.steps, front)
+            if a.dump_outputs:
+                dump_outputs(a.dump_outputs, r["outputs"])
             total_s, n = sum(r["times"]) / 1e3, len(r["times"])
             fps, cores = n / total_s, 2
             sample = (f"{n} published frames (2 images + 1 window solve each) of sequence seed 0 after {INIT_PUBS} init + {warmup} "
@@ -597,7 +634,7 @@ def main():
             n_seq_total = S * max(a.gpus, 1)
             procs_cap = max(1, (os.cpu_count() or 2) // 2)
             seeds = list(range(min(n_seq_total, procs_cap, n_distinct * max(a.gpus, 1))))
-            steps = min(a.steps, 20)
+            steps = a.steps
             res, wall, procs = run_reference_parallel(seeds, INIT_PUBS, warmup, steps, front)
             n = sum(x["n"] for x in res)
             # the pool's wall time contains start-up and the untimed init frames: use the slowest worker's timed region
@@ -649,7 +686,7 @@ def main():
     # frames are rendered (fork pool) before this process touches CUDA; the CPU-baseline sample needs a longer sequence
     cpu_frames = max(a.steps, a.cpu_frames) if (not a.no_cpu_baseline and world == 1 and not batched) else a.steps
     want_c3 = (batched or not a.no_c3)
-    c3_steps = min(a.steps, 20)
+    c3_steps = a.steps
     batch_inputs = None
     if want_c3:
         first_seed = 100 + shard.sequences_of_rank(rank, world, S)[0]
@@ -699,7 +736,7 @@ def main():
                "h2d_bytes_per_step": re_["h2d"] / max(re_["frames"], 1), "d2h_bytes_per_step": re_["d2h"] / max(re_["frames"], 1),
                "gpu_launches": rb["launches"], "clocks": clocks_b}
         if with_profile:
-            pr = run_batch_pass(batch_inputs, S, INIT_PUBS, 2, 6, local, profile=True)
+            pr = run_batch_pass(batch_inputs, S, INIT_PUBS, 2, min(6, warmup + c3_steps - 2), local, profile=True)
             kt = kernel_table(pr["trk_k"], pr["est_k"])
             n_solves = kt.get("ba_finish", {}).get("launches", 1)
             n_images = kt.get("pyrdown", {}).get("launches", 3) // 3
@@ -732,6 +769,8 @@ def main():
 
     if batched:
         rb, re_, obj = batch_object(with_profile=(rank == 0))
+        if a.dump_outputs and rank == 0:
+            dump_outputs(a.dump_outputs, rb["outputs"])
         fps_dev, t_dev, n_frames = shard.aggregate_rate(rb["region_ms"], rb["frames"], device=f"cuda:{local}")
         fps_e2e, t_e2e, _ = shard.aggregate_rate(re_["region_ms"], re_["frames"], device=f"cuda:{local}")
         launches = torch.tensor([float(rb["launches"])], device=f"cuda:{local}")
@@ -765,6 +804,8 @@ def main():
     clocks.start()
     res_dev = run_ours_pass(seq, ts, imgs, imu, INIT_PUBS, warmup, a.steps, local, host_images=False, flush=flush, sync_cb=rank_barrier,
                             clocks=clocks)
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, res_dev["outputs"])
     barrier()
     clk = clocks.stop()
     barrier()
@@ -779,7 +820,8 @@ def main():
     fps_e2e, t_e2e = agg(res_e2e)
 
     # ---- roofline of the dominant kernel, measured live with CUDA events in a profile pass
-    prof = run_ours_pass(seq, ts, imgs, imu, INIT_PUBS, 2, 10, local, host_images=False, profile=True)
+    # 2 warm-up + 10 profiled steps, fewer when the rendered sequence (sized for the timed passes) holds less
+    prof = run_ours_pass(seq, ts, imgs, imu, INIT_PUBS, 2, min(10, warmup + cpu_frames - 2), local, host_images=False, profile=True)
     kt = kernel_table(prof["trk_k"], prof["est_k"])
     n_solves = kt.get("ba_finish", {}).get("launches", 1)       # one double2vector launch per solve
     n_images = kt.get("pyrdown", {}).get("launches", 3) // 3      # three pyramid levels per image

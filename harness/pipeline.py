@@ -6,21 +6,35 @@ from __future__ import annotations
 
 import hashlib
 import os
+import tempfile
 
 import numpy as np
 
 from . import synth
 
 
-def cached_images(seq: synth.Sequence, n: int, cache_dir="/tmp/vinsb200_cache"):
-    os.makedirs(cache_dir, exist_ok=True)
+def cached_images(seq: synth.Sequence, n: int, cache_dir=None):
+    """The first n rendered images of seq, cached as .npy in a per-user directory under the system's temporary directory
+    (never in the source tree, which may be read-only).  A file appears under its final name only once it is complete, so
+    concurrent processes never read a partial one; a cache that cannot be written only costs the next call a render."""
+    if cache_dir is None:
+        cache_dir = os.path.join(tempfile.gettempdir(), f"vinsb200_cache-{os.getuid()}")
     key = hashlib.sha1(f"{seq.seed}-{seq.rows}x{seq.cols}-{seq.pixel_noise}-{seq.cam_hz}-{n}-v2".encode()).hexdigest()[:16]
     path = os.path.join(cache_dir, key + ".npy")
     ts = seq.image_times()[:n]
     if os.path.exists(path):
         return ts, np.load(path, mmap_mode="r")
     _, imgs = seq.images(n)
-    np.save(path, imgs)
+    tmp = None
+    try:
+        os.makedirs(cache_dir, mode=0o700, exist_ok=True)
+        fd, tmp = tempfile.mkstemp(dir=cache_dir, suffix=".partial")
+        with os.fdopen(fd, "wb") as f:
+            np.save(f, imgs)
+        os.replace(tmp, path)
+    except OSError:
+        if tmp is not None and os.path.exists(tmp):
+            os.unlink(tmp)
     return ts, imgs
 
 
